@@ -49,6 +49,7 @@ UNIT = "passes/s"
 LATENT = {"sdxl": 128, "sd15": 64}
 CTX_DIM = {"sdxl": 2048, "sd15": 768}
 KERNEL_CLASS = {"gemm": "gemm", "conv3x3": "gemm", "attention": "attention", "groupnorm": "norm", "layernorm": "norm"}
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def host_threads() -> int:
@@ -76,6 +77,24 @@ def host_threads() -> int:
     if env:
         n = int(env)
     return max(1, min(n, 64))  # MKL/oneDNN fp32 convs stop scaling (and start thrashing) well before 64 threads
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: each output of the last timed step as `<directory>/<name>.npy` in float32, so that two builds run
+    with the same arguments (hence the same seeded inputs) can be compared output for output.  When the outputs exceed
+    64 MiB in all, each array above an equal share of that is replaced by a fixed, seeded sample of its elements
+    (flattened, in index order; the indices depend only on the array's size)."""
+    import numpy as np
+
+    total = sum(4 * t.numel() for t in arrays.values())
+    cap = DUMP_LIMIT_BYTES // (4 * len(arrays)) if total > DUMP_LIMIT_BYTES else None
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().to("cpu", torch.float32)
+        if cap is not None and t.numel() > cap:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            t = t.reshape(-1)[idx]
+        np.save(os.path.join(directory, name + ".npy"), t.numpy())
 
 
 def load_peaks():
@@ -158,6 +177,7 @@ def build_product(dev, arch="sdxl", rank=4, seed=0, share=None):
         synthetic.init_synthetic_(unet, seed=seed + 1)
     unet.requires_grad_(False)
     unet.eval()
+    torch.manual_seed(seed)  # lora_down keeps its kaiming init, drawn from the global generator: same adaptors every run
     saved = list(plora.DEFAULT_TARGET_REPLACE)
     plora.DEFAULT_TARGET_REPLACE += plora.UNET_TARGET_REPLACE_MODULE_CONV  # c3lier (train_lora_xl.py:50-52)
     try:
@@ -252,6 +272,7 @@ def cpu_pair_call(arch="sdxl", rank=4, seed=0, lora_state=None, unet_state=None)
                             for k, p in om.named_parameters()}, assign=True)
     om.requires_grad_(False)
     om.eval()
+    torch.manual_seed(seed)  # the adaptors' kaiming init of lora_down: same weights every run
     if rb.available():
         lora, tu, mu = rb.load("lora"), rb.load("train_util"), rb.load("model_util")
         saved = list(lora.DEFAULT_TARGET_REPLACE)
@@ -292,18 +313,16 @@ def cpu_pair_call(arch="sdxl", rank=4, seed=0, lora_state=None, unet_state=None)
     return call, kind, what, (lat1, ehs, pooled, tids)
 
 
-def run_cpu_arm(steps, warmup, budget_s, threads):
+def run_cpu_arm(steps, warmup, threads):
     call, kind, what, _ = cpu_pair_call("sdxl")
     torch.set_num_threads(threads)
-    times, t_start = [], time.time()
+    times, eps = [], None
     for i in range(warmup + steps):
         t0 = time.time()
-        call()
+        eps = call()
         if i >= warmup:
             times.append(time.time() - t0)
-        if time.time() - t_start > budget_s and times:
-            break
-    return times, kind, what
+    return times, kind, what, eps
 
 
 def cpu_config1(threads):
@@ -341,7 +360,9 @@ def cpu_config1(threads):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline forward, e2e call, per-class graphs, SD-1.5 forwards (config 2) and "
+                         "the --impl reference arm; configs 3 and 4 time 3 iterations, config 5 one sweep")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--batch", type=int, default=8, help="conditioned passes per GPU per step")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
@@ -349,6 +370,8 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=30.0)
     ap.add_argument("--no-train", action="store_true", help="skip the training-iteration timings (configs 3 and 4)")
     ap.add_argument("--no-extra", action="store_true", help="skip BASELINE configs 1, 2 and 5")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of each timed path returned to DIR/<name>.npy (float32, rank 0)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(min(args.warmup, 1), 1)
 
@@ -366,12 +389,13 @@ def main():
         if rank != 0:
             return
         threads = host_threads()
-        times, kind, what = run_cpu_arm(args.steps, args.warmup, budget_s=240.0, threads=threads)
+        times, kind, what, eps = run_cpu_arm(args.steps, args.warmup, threads=threads)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"cpu_guided_eps": eps})
         ms = 1e3 * statistics.mean(times)
         v = 2.0 * 1e3 / ms                       # a CFG-pair call is two conditioned passes
         sample = (f"{len(times)} timed CFG-pair calls (predict_noise_xl, batch 1 = 2 passes each, guidance 3, rank-4 LoRA "
-                  f"hook live) of the same SDXL@128x128 workload, fp32, {threads} threads, 240 s budget "
-                  f"({args.steps} requested); {what}")
+                  f"hook live) of the same SDXL@128x128 workload, fp32, {threads} threads; {what}")
         print(json.dumps({"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus,
                           "steps": len(times), "steps_requested": args.steps, "warmup": args.warmup, "ms_per_step": ms,
                           "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -399,6 +423,19 @@ def main():
     lat, ehs = lat_h.to(dev), ehs_h.to(dev)
     added = {"text_embeds": pooled_h.to(dev), "time_ids": tids_h.to(dev)}
     fwd = lambda: unet(lat, 500, ehs, added_cond_kwargs=added).sample
+    dump, last = {}, {}   # --dump-outputs: what the last timed call of each path returned
+
+    def keep(name, fn):
+        if not args.dump_outputs:
+            return fn
+
+        def step():
+            last[name] = fn()
+        return step
+
+    def record(name, make):
+        if args.dump_outputs:
+            dump[name] = make()
 
     # ---- per-kernel-class graphs (also captures the whole-forward graph used below)
     net.__enter__()  # multiplier = 1 (lora.py:252-254)
@@ -407,8 +444,9 @@ def main():
 
         # ---- value: graph replay of the whole forward, inputs resident
         sampler = ClockSampler(local_rank)
-        ms_step = timed(fwd, args.steps, args.warmup, dm, sampler)
+        ms_step = timed(keep("sample", fwd), args.steps, args.warmup, dm, sampler)
         clocks = sampler.stop()
+        record("sdxl_fwd_sample", lambda: last["sample"].float().cpu())   # graph output buffer: copy before the next replay
     value = world * B / (ms_step * 1e-3)
     gm = classes.get("gemm", {"ms": 0.0, "launches": 0, "flops": 0.0})
     achieved = gm["flops"] / (gm["ms"] * 1e-3) / 1e12 if gm["ms"] > 0 else 0.0
@@ -451,6 +489,7 @@ def main():
 
     with torch.no_grad():
         e2e_ms = timed(e2e_step, args.steps, args.warmup, dm)
+    record("e2e_guided_eps", lambda: eps_host[:half].clone())
     h2d = (lat_h[:half].numel() * 4 + ehs_h[:2 * half].numel() * 2 + pooled_h[:2 * half].numel() * 2
            + tids_h[:2 * half].numel() * 4)
     e2e = {"value": world * 2 * half / (e2e_ms * 1e-3), "unit": UNIT, "h2d_bytes_per_step": h2d,
@@ -471,7 +510,8 @@ def main():
                                                    guidance_scale=5.0, start_noise=750)
         with torch.no_grad():
             sweep((1.0,), 2)                 # captures the two 32-pass graphs (adaptors gated off / on)
-            ms5 = timed(lambda: sweep(scales, 50), 1, 0)
+            ms5 = timed(keep("sweep", lambda: sweep(scales, 50)), 1, 0)
+        record("config5_sweep_latents", lambda: torch.stack([x.float().cpu() for x in last["sweep"]]))
         per_scale_s = ms5 * 1e-3 / len(scales)
         extra["config5_inference_sweep"] = {
             "what": "eval denoise loop (generate_images_xl.py:325-364): batch 16, CFG 5, 50 DDIM steps, slider gated on "
@@ -509,6 +549,7 @@ def main():
 
         n_it = 3
         it_ms = timed(text_it, n_it, 1, dm)
+        record("config3_text_slider_loss", lambda: torch.tensor([float(state["loss"])]))
         parallel.assert_replicas_equal(list(net.parameters()), sgroup)
         passes = 2 * (25 + 4)  # CFG pairs: 25 denoise steps + positive / neutral / unconditional / target
         gw = world // n_sliders  # ranks per slider
@@ -544,6 +585,7 @@ def main():
                                                     timesteps_to=20, seed=4, device=dev, weight_dtype=torch.bfloat16)
 
         im_ms = timed(image_it, n_it, 1, dm)
+        record("config4_image_slider_losses", lambda: torch.tensor([float(x) for x in st4["l"]]))
         parallel.assert_replicas_equal(list(net8.parameters()))
         extra["config4_image_slider"] = {
             "what": "BASELINE config 4 — image-slider step, SDXL, rank-8 LoRA, paired synthetic latents [1,4,128,128] with shared "
@@ -565,7 +607,8 @@ def main():
             for b in (1, 2, 8):
                 l15, e15, _, _ = make_host_inputs(b, "sd15", seed=b, pin=False)
                 l15, e15 = l15.to(dev), e15.to(dev)
-                ms15 = timed(lambda: u15(l15, 500, e15).sample, args.steps, args.warmup)
+                ms15 = timed(keep("sd15", lambda: u15(l15, 500, e15).sample), args.steps, args.warmup)
+                record(f"config2_sd15_fwd_sample_B{b}", lambda: last["sd15"].float().cpu())
                 pps = b / (ms15 * 1e-3)
                 rows[f"B{b}"] = {"ms_per_forward": ms15, "passes_per_s": pps,
                                  "frac_of_sustained": pps * (FLOPS_PER_PASS["sd15"] + FLOPS_LORA[("sd15", 4)]) / 1e12 / peaks["sustained"]}
@@ -613,6 +656,8 @@ def main():
                 "launches_per_step": launches_per_fwd, "roofline": roofline, "cpu_baseline": cpu_baseline,
                 "train": train, "configs": extra}
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dump)
     if world > 1:
         dist.destroy_process_group()
 

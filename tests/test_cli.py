@@ -1,18 +1,18 @@
 """CPU tests of the trainers' command line (sliders_b200/cli.py, config_util.py, prompt_util.py, model_util.py): the YAML
-schema and the flag semantics of the reference's train_lora*.py, checked against the reference's own config_util /
-prompt_util modules where /root/reference exists (this container; the GPU box skips those)."""
+schema and the flag semantics of the reference's train_lora*.py, checked against what the reference's own config_util /
+prompt_util modules make of the reference's data files (tests/golden/make_golden_reference.py)."""
 import os
 import sys
 
 import pytest
 import torch
 
-from oracle import reference_bridge as rb
 from sliders_b200 import cli, config_util, model_util, prompt_util
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DATA = os.path.join(ROOT, "trainscripts", "textsliders", "data")
-needs_ref = pytest.mark.skipif(not rb.available(), reason="reference tree not present")
+GOLDEN = os.path.join(ROOT, "tests", "golden")
+REF_DATA = os.path.join(GOLDEN, "reference_data")   # the reference's own data files, verbatim
 
 
 def test_shipped_yaml_parses_and_builds_pairs():
@@ -82,19 +82,15 @@ def test_model_sources():
         assert model_util.create_noise_scheduler(name) is not None
 
 
-@needs_ref
 def test_reference_yaml_files_parse_like_the_reference():
-    rc, rp = rb.load("config_util"), rb.load("prompt_util")
-    ref_dir = os.path.join(rb.REFERENCE_ROOT, "trainscripts", "textsliders", "data")
+    ref = torch.load(os.path.join(GOLDEN, "reference_calls.pt"))["yaml"]   # the reference parsers' `.dict()`
     for name in ("config-xl.yaml", "config.yaml"):
-        ours = config_util.load_config_from_yaml(os.path.join(ref_dir, name))
-        ref = rc.load_config_from_yaml(os.path.join(ref_dir, name))
-        assert ours.model_dump() == ref.dict()
+        ours = config_util.load_config_from_yaml(os.path.join(REF_DATA, name))
+        assert ours.model_dump() == ref[name]
     for name, atts in (("prompts-xl.yaml", ["male", "female"]), ("prompts.yaml", []),
                        ("prompts-person_age_slider_GPT.yaml", ["asian", "white"])):
-        ours = prompt_util.load_prompts_from_yaml(os.path.join(ref_dir, name), atts)
-        ref = rp.load_prompts_from_yaml(os.path.join(ref_dir, name), atts)
-        assert [o.model_dump() for o in ours] == [r.dict() for r in ref]
+        ours = prompt_util.load_prompts_from_yaml(os.path.join(REF_DATA, name), atts)
+        assert len(ref[name]) > 0 and [o.model_dump() for o in ours] == ref[name]
 
 
 def test_eval_sweep_host_logic(tmp_path):
@@ -111,6 +107,5 @@ def test_eval_sweep_host_logic(tmp_path):
     assert torch.equal(a, torch.randn(2, 4, 8, 8) * 2.0)      # == generator = torch.manual_seed(seed) + prepare_latents
     args = es.build_parser().parse_args(["--model_name", "m.pt", "--prompts_path", "p.csv", "--save_path", "o"])
     assert (args.start_noise, args.rank, args.num_samples, args.ddim_steps) == (750, 4, 1, 50)
-    if rb.available():                                        # the reference's own prompt files have these columns
-        ref = es.read_prompts_csv(os.path.join(rb.REFERENCE_ROOT, "prompts", "prompts-person.csv"))
-        assert len(ref) > 10 and ref[0]["prompt"] == "image of a person"
+    ref = es.read_prompts_csv(os.path.join(REF_DATA, "prompts-person.csv"))   # the reference's own prompt file
+    assert len(ref) > 10 and ref[0]["prompt"] == "image of a person"

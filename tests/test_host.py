@@ -2,6 +2,8 @@
 module tree / LoRANetwork mirror the reference interface, the product DDIM scheduler agrees with the oracle
 restatement, checkpoints round-trip in the reference layout, and the multi-rank fan-out helpers reproduce the
 single-rank result under gloo with world_size 2.  No GPU compute happens here."""
+import gzip
+import json
 import os
 import re
 import subprocess
@@ -12,11 +14,11 @@ import torch
 
 from conftest import c3lier
 from oracle import ddim as oddim
-from oracle import reference_bridge as rb
 from sliders_b200 import _cabi, lora as plora, parallel, scheduler as psched, synthetic
 from sliders_b200.unet import UNet2DConditionModel, UNetConfig
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 
 # ---------------------------------------------------------------------------------------- C ABI
@@ -130,14 +132,12 @@ def test_checkpoint_roundtrip_pt_and_safetensors(tmp_path):
         assert not missing.missing_keys and not missing.unexpected_keys
         for k, v in net.state_dict().items():
             assert torch.equal(net2.state_dict()[k].to(torch.bfloat16), v.to(torch.bfloat16)), k
-    if rb.available():  # a slider written by us loads into the reference's own LoRANetwork on the oracle UNet
-        from oracle import unet as ounet
-
-        rlora = rb.load("lora")
-        om = ounet.UNet2DConditionModel(ounet.UNetConfig(**cfg.__dict__))
-        with c3lier(rlora):
-            rnet = rlora.LoRANetwork(om, rank=4, multiplier=1.0, alpha=1.0, train_method="noxattn")
-        rnet.load_state_dict(torch.load(str(tmp_path / "slider_alpha1.0_rank4_noxattn_last.pt")), strict=True)
+    # a slider written by us loads strictly into the reference's own LoRANetwork on the oracle UNet: exactly its keys,
+    # each with its shape (tests/golden/make_golden_reference.py records them)
+    with gzip.open(os.path.join(GOLDEN, "reference_lora_keys.json.gz"), "rt") as f:
+        ref = json.load(f)["small_unet_checkpoint"]
+    sd = torch.load(str(tmp_path / "slider_alpha1.0_rank4_noxattn_last.pt"))
+    assert {k: list(v.shape) for k, v in sd.items()} == ref
 
 
 # ---------------------------------------------------------------------------------------- scheduler
@@ -303,24 +303,19 @@ def test_prompt_pair_loss_and_optimizer_factory():
 
 
 def test_reference_prompt_pair_loss_matches_ours():
-    from oracle import reference_bridge as rb
-
-    if not rb.available():
-        pytest.skip("/root/reference not present (GPU box)")
+    """Against the reference's PromptEmbedsPair (prompt_util.py) on the same latents (golden, reference_calls.pt)."""
     from sliders_b200 import trainer
 
-    pu = rb.load("prompt_util")
-    g = torch.Generator().manual_seed(1)
-    t, p, u, n = (torch.randn(2, 4, 8, 8, generator=g) for _ in range(4))
+    fx = torch.load(os.path.join(GOLDEN, "reference_calls.pt"))["prompt_pair"]
+    t, p, u, n = fx["target"], fx["positive"], fx["unconditional"], fx["neutral"]
     for action in ("erase", "enhance"):
-        rs = pu.PromptSettings(target="t", positive="p", unconditional="u", neutral="n", action=action,
-                               guidance_scale=2.5, resolution=512, batch_size=2)
-        ref = pu.PromptEmbedsPair(torch.nn.MSELoss(), None, None, None, None, rs)
+        ref = fx[action]
         ours = trainer.PromptEmbedsPair(torch.nn.MSELoss(), None, None, None, None,
-                                        trainer.PromptSettings(guidance_scale=2.5, action=action, batch_size=2))
+                                        trainer.PromptSettings(guidance_scale=fx["guidance_scale"], action=action,
+                                                               batch_size=fx["batch_size"]))
         kw = dict(target_latents=t, positive_latents=p, unconditional_latents=u, neutral_latents=n)
-        assert torch.equal(ref.loss(**kw), ours.loss(**kw))
-        assert (ref.batch_size, ref.resolution, ref.dynamic_crops) == (ours.batch_size, 512, ours.dynamic_crops)
+        assert torch.equal(ref["loss"], ours.loss(**kw))
+        assert (ref["batch_size"], ref["resolution"], ref["dynamic_crops"]) == (ours.batch_size, 512, ours.dynamic_crops)
 
 
 _TRAIN_WORKER = r'''

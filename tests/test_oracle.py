@@ -1,7 +1,8 @@
 """CPU tests that pin the oracle (oracle/unet.py, oracle/ddim.py) — the reference has no tests of its own
-(SURVEY.md §4), so the restatement is pinned by known answers of the published architecture, by the golden
-vectors produced with the reference's own unmodified lora.py / train_util.py (tests/golden/make_golden.py) and,
-when /root/reference is present, by running those reference modules live."""
+(SURVEY.md §4), so the restatement is pinned by known answers of the published architecture and by the golden
+vectors produced with the reference's own unmodified lora.py / train_util.py (tests/golden/make_golden*.py)."""
+import gzip
+import json
 import os
 
 import pytest
@@ -9,12 +10,17 @@ import torch
 
 from conftest import c3lier
 from oracle import ddim as oddim
-from oracle import reference_bridge as rb
+from oracle import port
 from oracle import unet as ounet
 from sliders_b200 import synthetic
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
-needs_ref = pytest.mark.skipif(not rb.available(), reason="/root/reference not present (GPU box)")
+
+
+def _reference_lora_keys():
+    """What the reference's LoRANetwork (lora.py) builds on the oracle UNet (tests/golden/make_golden_reference.py)."""
+    with gzip.open(os.path.join(GOLDEN, "reference_lora_keys.json.gz"), "rt") as f:
+        return json.load(f)
 
 
 # ---------------------------------------------------------------------------------------- structure KATs
@@ -46,24 +52,26 @@ def test_hf_key_names():
     assert sd1.state_dict()["down_blocks.0.attentions.0.proj_in.weight"].shape == (320, 320, 1, 1)  # conv projection
 
 
-@needs_ref
 @pytest.mark.parametrize("name,n_leaves,n_params,rank", [("sdxl", 346, 4_320_000, 4), ("sdxl", 346, 8_640_000, 8),
                                                          ("sd15", 150, 2_906_880, 4)])
 def test_reference_lora_injection_counts(name, n_leaves, n_params, rank):
-    lora = rb.load("lora")
-    with torch.device("meta"):
-        m = ounet.UNet2DConditionModel(getattr(ounet.UNetConfig, name)())
-        with c3lier(lora):
-            net = lora.LoRANetwork(m, rank=rank, multiplier=1.0, alpha=1.0, train_method="noxattn")
-    assert len(net.unet_loras) == n_leaves
-    assert sum(p.numel() for p in net.parameters()) == n_params
-    names = {l.lora_name for l in net.unet_loras}
+    """The reference's LoRANetwork finds the published adaptor set on the oracle UNet, and the CPU port of its hook
+    (oracle/port.py) finds the same leaves in the same order."""
+    ref = _reference_lora_keys()["counts"][f"{name}/{rank}"]
+    assert ref["n_leaves"] == n_leaves and len(ref["lora_names"]) == n_leaves
+    assert ref["n_params"] == n_params
+    names = set(ref["lora_names"])
     for k in ("lora_unet_down_blocks_0_resnets_0_conv1", "lora_unet_down_blocks_0_resnets_0_time_emb_proj",
               "lora_unet_down_blocks_0_downsamplers_0_conv", "lora_unet_up_blocks_2_resnets_2_conv_shortcut",
               "lora_unet_mid_block_attentions_0_transformer_blocks_0_attn1_to_out_0"):
         if name == "sdxl":
             assert k in names, k
     assert not any("attn2" in n for n in names)
+    with torch.device("meta"):
+        m = ounet.UNet2DConditionModel(getattr(ounet.UNetConfig, name)())
+        net = port.LoRAHooks(m, rank=rank, alpha=1.0, c3lier=True)
+    assert [l.lora_name for l in net.unet_loras] == ref["lora_names"]
+    assert sum(p.numel() for p in net.parameters()) == n_params
 
 
 # ---------------------------------------------------------------------------------------- scheduler KATs
@@ -191,59 +199,62 @@ def test_golden_loss_formula():
     assert torch.allclose(want, fx["loss_enhance_g4"], rtol=1e-5)
 
 
-# ---------------------------------------------------------------------------------------- live reference
-@needs_ref
+# ---------------------------------------------------------------------------------------- reference LoRA interface
 def test_zero_init_identity_and_multiplier_semantics_with_reference_lora():
-    lora = rb.load("lora")
-    tu = rb.load("train_util")
-    mu = rb.load("model_util")
-    m = _tiny("tiny_xl")
+    """Identity and multiplier semantics of the LoRA hook through predict_noise_xl, run by the CPU port of hook + call on
+    the oracle UNet, and the port's outputs against those of the reference's own code on the same weights and inputs
+    (golden, reference_calls.pt)."""
+    fx = torch.load(os.path.join(GOLDEN, "reference_calls.pt"))["hook_xl"]
+    m = _tiny("tiny_xl", seed=fx["weight_seed"])
     m.requires_grad_(False)
-    g = torch.Generator().manual_seed(5)
+    g = torch.Generator().manual_seed(fx["input_seed"])
     lat = torch.randn(1, 4, 16, 16, generator=g)
     ehs = torch.randn(2, 77, 256, generator=g)
     pooled = torch.randn(2, 128, generator=g)
     tids = torch.tensor([[128., 128, 0, 0, 128, 128]] * 2)
-    sched = mu.create_noise_scheduler("ddim")
+    t = fx["timestep"]
+    sched = _ddim()
     sched.set_timesteps(1000)
+
+    def close(a, b):
+        return ((a - b).norm() / b.norm()).item() < 1e-5
+
     with torch.no_grad():
-        base = tu.predict_noise_xl(m, sched, 500, lat, ehs, pooled, tids, guidance_scale=1)
-        with c3lier(lora):
-            net = lora.LoRANetwork(m, rank=4, multiplier=1.0, alpha=1.0, train_method="noxattn")
-        with net:  # fresh LoRA: lora_up == 0  ->  identity (lora.py:97-98)
-            fresh = tu.predict_noise_xl(m, sched, 500, lat, ehs, pooled, tids, guidance_scale=1)
+        base = port.predict_noise_xl(m, sched, t, lat, ehs, pooled, tids, guidance_scale=1)
+        assert close(base, fx["base"])
+        net = port.LoRAHooks(m, rank=fx["rank"], alpha=fx["alpha"], c3lier=True)
+        with net:  # fresh LoRA: lora_up == 0 -> identity (lora.py:97-98)
+            fresh = port.predict_noise_xl(m, sched, t, lat, ehs, pooled, tids, guidance_scale=1)
         assert torch.equal(fresh, base)
-        synthetic.init_lora_nonzero_(net, seed=1, up_std=0.05)
-        off = tu.predict_noise_xl(m, sched, 500, lat, ehs, pooled, tids, guidance_scale=1)  # multiplier 0 after exit
+        synthetic.init_lora_nonzero_(net, seed=fx["lora_seed"], up_std=fx["up_std"], reseed_down=True)
+        off = port.predict_noise_xl(m, sched, t, lat, ehs, pooled, tids, guidance_scale=1)  # multiplier 0 after exit
         assert torch.allclose(off, base, atol=1e-6)
         with net:
-            on = tu.predict_noise_xl(m, sched, 500, lat, ehs, pooled, tids, guidance_scale=1)
+            on = port.predict_noise_xl(m, sched, t, lat, ehs, pooled, tids, guidance_scale=1)
         assert (on - base).abs().max() > 1e-3
-        # guidance_scale = 1  =>  guided == text half (train_util.py:250-253)
-        out = m(torch.cat([lat] * 2), 500, ehs, added_cond_kwargs={"text_embeds": pooled, "time_ids": tids}).sample
+        assert close(on, fx["on"])
+        # guidance_scale = 1 => guided == text half (train_util.py:250-253)
+        out = m(torch.cat([lat] * 2), t, ehs, added_cond_kwargs={"text_embeds": pooled, "time_ids": tids}).sample
         assert torch.allclose(base, out.chunk(2)[1], atol=1e-6)
 
 
-@needs_ref
 def test_reference_state_dict_keys_match_ours():
     from sliders_b200 import lora as plora
     from sliders_b200.unet import UNet2DConditionModel as PU, UNetConfig as PC
 
-    lora = rb.load("lora")
-    for cfg_o, cfg_p in ((ounet.UNetConfig.sdxl(), PC.sdxl()), (ounet.UNetConfig.sd15(), PC.sd15())):
+    ref_keys = _reference_lora_keys()["state_dict_keys"]
+    for name, cfg_o, cfg_p in (("sdxl", ounet.UNetConfig.sdxl(), PC.sdxl()), ("sd15", ounet.UNetConfig.sd15(), PC.sd15())):
         with torch.device("meta"):
             mo, mp = ounet.UNet2DConditionModel(cfg_o), PU(cfg_p)
             assert list(mo.state_dict().keys()) == list(mp.state_dict().keys())
             assert [tuple(v.shape) for v in mo.state_dict().values()] == [tuple(v.shape) for v in mp.state_dict().values()]
             for method in ("noxattn", "full", "xattn", "selfattn", "innoxattn", "xattn-strict", "noxattn-hspace",
                            "noxattn-hspace-last"):
-                with c3lier(lora):
-                    a = lora.LoRANetwork(mo, rank=4, multiplier=1.0, alpha=1.0, train_method=method)
                 with c3lier(plora):
                     b = plora.LoRANetwork(mp, rank=4, multiplier=1.0, alpha=1.0, train_method=method)
-                assert list(a.state_dict().keys()) == list(b.state_dict().keys()), method
-                # re-create fresh models: injection swaps the leaf forwards
-                mo, mp = ounet.UNet2DConditionModel(cfg_o), PU(cfg_p)
+                assert list(b.state_dict().keys()) == ref_keys[f"{name}/{method}"], method
+                # re-create a fresh model: injection swaps the leaf forwards
+                mp = PU(cfg_p)
 
 
 def test_euler_discrete_known_answers_and_ddim_equivalence():
